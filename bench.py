@@ -2,7 +2,7 @@
 """Benchmark of the hot path: ray-samples/s on BASELINE.json's configs.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--pass step|forward] [--config c2|c3|c4|c5] [--with-eikonal]
-                  [--precision fp16x3|fp16|bf16]
+                  [--precision fp16x3|fp16|bf16] [--dump-outputs DIR]
 
 Default = configs[1] (C2): fg-bob deformable field, 2048 rays x 128 samples per GPU, synthetic rays and synthetic
 "trained-like" weights, ONE TRAINING STEP of the renderer per "step":
@@ -170,10 +170,28 @@ def make_problem(device, rank, field, M, N, D, n_inst=1):
     return out
 
 
+def dump_outputs(path, rend, renderers, train, limit=64 << 20):
+    """Write what one step of the timed path hands its caller - the rendered pixels and, for a training step, every hot-path
+    parameter's gradient (per field) - as float32 DIR/<name>.npy.  An array larger than its equal share of `limit` bytes is
+    replaced by a fixed sample of its flattened elements (seeded by the array's size, so two runs pick the same ones)."""
+    arrs = {f"rend.{k}": v for k, v in sorted(rend.items())}
+    if train:
+        for fi, r in enumerate(renderers):
+            arrs.update({f"grad.{fi}.{k}": v for k, v in r.grad_buffer()[1].items()})
+    share = limit // (4 * len(arrs))
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrs.items():
+        a = t.detach().float().cpu()
+        if a.numel() > share:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(a.numel()))[:share].sort().values
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(path, name + ".npy"), a.numpy())
+
+
 # ------------------------------------------------------------------------------------------ CPU arm (reference's PyTorch path)
 def cpu_reference_rate(field, M, N, D, with_backward, reps, threads):
-    """The reference's CPU PyTorch implementation of the path on the host cores: the UNMODIFIED reference (baseline/_ref
-    through oracle/ref_shims) when the travelling copy is present, else the oracle port."""
+    """The reference's CPU PyTorch implementation of the path on the host cores: the UNMODIFIED reference (oracle/_ref
+    through oracle/ref_shims) when that copy is present, else the oracle port."""
     torch.set_num_threads(threads)
     kind = "port"
     try:
@@ -350,7 +368,11 @@ def main():
                     help="the step also evaluates the eikonal term on 1/16 of the rays (reverse chain, loss, forward chains + weight gradients: "
                          "NeRF.compute_eikonal and its second-order backward)")
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of replaying the step as a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's rendered outputs and parameter gradients to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -388,14 +410,16 @@ def main():
         return rend
 
     def timed(fn, steps):
+        """Per-step times (ms) of `steps` calls of fn, and what the last call returned."""
         ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(steps)]
+        out = None
         for i in range(steps):
             flush.fill_(i & 0xFF)  # evict L2 between timed iterations
             ev[i][0].record()
-            fn()
+            out = fn()
             ev[i][1].record()
         torch.cuda.synchronize()
-        return [a.elapsed_time(b) for a, b in ev]
+        return [a.elapsed_time(b) for a, b in ev], out
 
     for _ in range(args.warmup):
         step.run()
@@ -423,13 +447,15 @@ def main():
     launches_per_step = step.launches
     torch.cuda.synchronize()
     t_wall0 = time.perf_counter()
-    ms = timed(run_fn, args.steps)
+    ms, last_rend = timed(run_fn, args.steps)
     n_launch = launches_per_step * args.steps
     torch.cuda.synchronize()
     if world > 1:
         dist.barrier()
     t_wall = time.perf_counter() - t_wall0
-    ms_e2e = timed(e2e_fn, args.steps)
+    if args.dump_outputs and rank == 0:  # before the end-to-end arm's steps overwrite the gradient buffers
+        dump_outputs(args.dump_outputs, last_rend, step.renderers, step.train)
+    ms_e2e, _ = timed(e2e_fn, args.steps)
     # the phases alone: the forward call and the backward call of the (last) field, each replayed as its own CUDA graph and
     # timed with CUDA events on the launching stream
     phase = {"fwd_ms": [], "bwd_ms": []}
@@ -509,7 +535,7 @@ def main():
                     return render_pixel(ft, dl)
 
                 gfo = GraphedStep(fwd_only, warmup=2, device=device)
-                tms = timed(gfo.replay, 20)
+                tms, _ = timed(gfo.replay, 20)
                 fwd_variants[prec] = {"ms_per_step": float(np.mean(tms)), "value_per_gpu": step.S / (float(np.mean(tms)) * 1e-3), "unit": "ray-samples/s",
                                       "what": "pack + query_field + render_pixel, no tape"}
                 gfo = None
@@ -527,7 +553,7 @@ def main():
             for _ in range(3):
                 st2.run()
             g2 = GraphedStep(st2.run, warmup=2, device=device)
-            tms = timed(g2.replay, 30)
+            tms, _ = timed(g2.replay, 30)
             step_variants["with_eikonal"] = {"ms_per_step": float(np.mean(tms)), "value_per_gpu": st2.S / (float(np.mean(tms)) * 1e-3), "unit": "ray-samples/s",
                                              "what": "the default step + NeRF.compute_eikonal on 1/16 of the rays and its second-order backward (eikonal kernels)"}
             g2 = st2 = None
@@ -616,18 +642,13 @@ def main():
                                     "sample": f"{reps} x ({Ms} of {cfgd['M']} frames x {step.N} rays x {step.D} samples), "
                                               f"{'forward+backward' if step.train else 'forward'}, fp32, {reps * dt:.1f} s"}
         print(json.dumps(line), flush=True)
-    # tear-down: graphs that captured NCCL collectives must go before the process group does; a stuck communicator
-    # tear-down must never outlive the measurement (the line above is already out)
+    # tear-down: graphs that captured NCCL collectives must go before the process group does; then an ordinary interpreter
+    # exit (exit handlers and library destructors run)
     g_run = g_e2e = gf = gb = run_fn = e2e_fn = f_fn = b_fn = None
     torch.cuda.synchronize()
     if world > 1:
-        try:
-            dist.barrier()
-        except Exception:
-            pass
-    sys.stdout.flush()
-    sys.stderr.flush()
-    os._exit(0)
+        dist.barrier()
+        dist.destroy_process_group()
 
 
 if __name__ == "__main__":

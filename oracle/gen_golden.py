@@ -121,6 +121,51 @@ def one_importance(name, motion, M, N, D, seed=0):
     print(name, "->", os.path.getsize(path) // 1024, "KiB; depth range", float(depth.min()), float(depth.max()))
 
 
+def reference_checks():
+    """tests/golden/reference/checks.npz: the reference's own results on the seeded inputs of three tests - dvr_model's
+    reconstruction losses (tests/test_loss_oracle_cpu.py), FeatureNeRF.global_match (tests/test_match_oracle_cpu.py) and
+    quat_transform.quaternion_apply with its gradients (tests/test_gpu_quat.py).  A subdirectory: the field fixtures are every
+    tests/golden/*.npz."""
+    import copy
+
+    sys.path.insert(0, os.path.join(HERE, "..", "tests"))
+    import types
+
+    import lab4d.utils.quat_transform as qt
+    from lab4d.engine.model import dvr_model
+    from lab4d.nnutils.feature import FeatureNeRF
+    from test_gpu_quat import quat_apply_inputs
+    from test_loss_oracle_cpu import CONFIG, synth_loss_inputs
+    from test_match_oracle_cpu import CANDIDATES, match_inputs
+
+    pack = {}
+    for ft in ("fg", "bg", "comp"):
+        rendered, aux, batch = synth_loss_inputs(ft)
+        config = dict(CONFIG, field_type=ft)
+        results = {"rendered": copy.deepcopy(rendered), "aux_dict": copy.deepcopy(aux)}
+        if "fg" in aux:  # the reference reads gauss_mask from aux (render_samples puts every field's rendering there)
+            results["aux_dict"]["fg"]["gauss_mask"] = results["rendered"]["gauss_mask"]
+        ref = {}
+        dvr_model.compute_recon_loss(ref, results, batch, config)
+        dvr_model.mask_losses(ref, batch, config)
+        dvr_model.apply_loss_weights(ref, config)
+        pack[f"loss/{ft}/keys"] = np.array(list(ref))
+        for k, v in ref.items():
+            pack[f"loss/{ft}/{k}"] = v.detach().numpy()
+    feat_px, feat_can, xyz, logsigma = match_inputs()
+    for K in CANDIDATES:
+        torch.manual_seed(5)
+        pack[f"match/K{K}"] = FeatureNeRF.global_match(types.SimpleNamespace(logsigma=logsigma), feat_px, feat_can, xyz, num_candidates=K).numpy()
+    q, p = (t.requires_grad_(True) for t in quat_apply_inputs())
+    out = qt.quaternion_apply(q.expand(5, 7, 4), p)
+    gq, gp = torch.autograd.grad(out.square().sum(), (q, p))
+    pack.update({"quat_apply/out": out.detach().numpy(), "quat_apply/gq": gq.numpy(), "quat_apply/gp": gp.numpy()})
+    path = os.path.join(OUT, "reference", "checks.npz")
+    os.makedirs(os.path.dirname(path), exist_ok=True)
+    np.savez_compressed(path, **pack)
+    print(path, "->", os.path.getsize(path) // 1024, "KiB")
+
+
 if __name__ == "__main__":
     os.makedirs(OUT, exist_ok=True)
     one("bg_rigid_M2_N16_D16", "bg", "rigid", 2, 16, 16)
@@ -131,3 +176,4 @@ if __name__ == "__main__":
     one("fg_compquad_M4_N8_D16", "fg", "comp_skel-quad_dense", 4, 8, 16, seed=3)
     one("fg_skelhuman_M4_N8_D24", "fg", "skel-human", 4, 8, 24, seed=4)
     one_importance("imp_fg_bob_M2_N8_D32", "bob", 2, 8, 32, seed=5)
+    reference_checks()

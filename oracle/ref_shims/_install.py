@@ -15,10 +15,10 @@ import torch
 
 import os
 
-# The reference checkout when it exists (build container), else the git-ignored copy that travels to the GPU box
-# (baseline/_ref, written by tools/make_ref.py / __graft_entry__.build()).
+# The reference checkout when it exists, else the git-ignored copy of its package
+# (oracle/_ref, written by oracle/make_ref.py / __graft_entry__.build()).
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_REF_COPY = os.path.normpath(os.path.join(_HERE, "..", "..", "baseline", "_ref"))
+_REF_COPY = os.path.normpath(os.path.join(_HERE, "..", "_ref"))
 REF_ROOT = os.environ.get("LAB4D_REF_ROOT") or ("/root/reference" if os.path.isdir("/root/reference/lab4d") else _REF_COPY)
 
 

@@ -1,13 +1,15 @@
-"""CPU, build container only (needs /root/reference): the drop-in adapter reads the architecture and the
-per-frame tables out of live reference modules exactly as the golden-vector harness does."""
+"""CPU: the drop-in adapter reads the architecture and the per-frame tables out of live reference modules exactly as the
+golden-vector harness does.  Needs the reference's lab4d package (a reference checkout, or its copy under oracle/_ref/)."""
 import os
 import sys
 
 import pytest
 import torch
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "ref_shims"))
+import _install  # noqa: E402
+
+pytestmark = pytest.mark.skipif(not _install.available(), reason="the reference's lab4d package is not present (oracle/_ref/)")
 
 
 def test_adapter_reads_reference_modules():

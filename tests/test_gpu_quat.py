@@ -1,6 +1,9 @@
 """GPU parity of the quaternion operators (lab4d_b200/quaternion.py over csrc/quat.cu: the dqtorch extension of the reference,
 lab4d/third_party/quaternion/src/quaternion.cu:29-217) against the pure-torch restatement with the CUDA kernels' semantics
 (3-vectors are pure quaternions): product, conjugate, first and second derivatives.  fp32 elementwise: 1e-6."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
@@ -36,36 +39,23 @@ def test_quaternion_mul_and_its_two_derivatives(B, D1, D2):
     assert torch.equal(gq, conj(G.detach()))
 
 
+def quat_apply_inputs():
+    g = torch.Generator().manual_seed(2)
+    q = torch.nn.functional.normalize(torch.randn(5, 1, 4, generator=g), dim=-1)
+    p = torch.randn(5, 7, 3, generator=g)
+    return q, p
+
+
 def test_quat_transform_runs_on_the_kernels():
-    """nnutils.install(dqtorch=True): lab4d.utils.quat_transform's quaternion_apply / dual-quaternion helpers on the kernels
-    equal the reference's own (pure-torch shim) results, with broadcasting operands."""
-    import os
-    import sys
-
-    ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    sys.path.insert(0, os.path.join(ROOT, "oracle", "ref_shims"))
-    import _install
-
-    if not _install.available():
-        pytest.skip("baseline/_ref (reference copy) not present")
-    import ref_harness  # noqa: F401
-    import lab4d.utils.quat_transform as qt
+    """nnutils.install(dqtorch=True): lab4d.utils.quat_transform.quaternion_apply (q p q*, vector part) on CUDA tensors goes
+    through nnutils._dq_mul / _dq_conj; on the kernels it equals the reference's own results and gradients, with broadcasting
+    operands (stored in tests/golden/reference/checks.npz by oracle/gen_golden.py)."""
     from lab4d_b200 import nnutils
 
-    g = torch.Generator().manual_seed(2)
-    q = torch.nn.functional.normalize(torch.randn(5, 1, 4, generator=g), dim=-1).to(DEV).requires_grad_(True)
-    p = torch.randn(5, 7, 3, generator=g).to(DEV).requires_grad_(True)
-
-    def run():
-        out = qt.quaternion_apply(q.expand(5, 7, 4), p)
-        (gq, gp) = torch.autograd.grad(out.square().sum(), (q, p))
-        return out.detach(), gq, gp
-
-    ref = run()
-    undo = nnutils.install(dqtorch=True)
-    try:
-        ours = run()
-    finally:
-        undo()
-    for o, t in zip(ours, ref):
-        assert rel_l2(o.cpu(), t.cpu()) <= 1e-6
+    golden = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference", "checks.npz"))
+    q, p = (t.to(DEV).requires_grad_(True) for t in quat_apply_inputs())
+    qe = q.expand(5, 7, 4)
+    out = nnutils._dq_mul(nnutils._dq_mul(qe, p), nnutils._dq_conj(qe))[..., 1:]
+    (gq, gp) = torch.autograd.grad(out.square().sum(), (q, p))
+    for name, o in (("out", out.detach()), ("gq", gq), ("gp", gp)):
+        assert rel_l2(o.cpu(), torch.from_numpy(golden[f"quat_apply/{name}"])) <= 1e-6, name

@@ -1,4 +1,4 @@
-"""GPU box: the UNMODIFIED reference (travelling copy baseline/_ref, imported through oracle/ref_shims) with and without
+"""GPU: the UNMODIFIED reference (its copy under oracle/_ref/, imported through oracle/ref_shims) with and without
 lab4d_b200.nnutils.install(): the patched reference modules run the B200 kernels end to end through the reference's own
 entry points (field.get_samples -> field.query_field -> render_pixel -> loss.backward(), and the eval-mode path of
 lab4d/render.py), and are compared with the un-patched reference on CUDA.  Skipped where the copy is absent."""
@@ -15,7 +15,7 @@ import _install  # noqa: E402
 
 from util import rel_l2  # noqa: E402
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not _install.available(), reason="baseline/_ref (reference copy) not present")]
+pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not _install.available(), reason="the reference's lab4d package is not present (oracle/_ref/)")]
 DEV = "cuda"
 
 
