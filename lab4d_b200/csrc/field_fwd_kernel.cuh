@@ -54,6 +54,8 @@ constexpr int kArenaGroup = 2 * kAChunkBytes;           // CH_PE, CH_EXTRA
 constexpr int kSmemArena = kGroups * kArenaGroup;        // 64 KB
 constexpr int kSmemRing = kNumStages * kWStageBytes;     // 96 KB
 constexpr int kTmemAcc = 0, kTmemAct = 256, kTmemGroup = 128;
+constexpr int kBarBytes = 256;                            // mbarriers + TMEM slot
+constexpr int kSdfPartBytes = 2 * 4 * kTileRows * 4;      // SPLIT: 8 partial sdf sums per row
 
 struct Q4 { float w, x, y, z; };
 __device__ __forceinline__ Q4 qmul(const Q4& a, const Q4& b) {
@@ -97,9 +99,12 @@ using IC = std::integral_constant<int, V>;
 
 // SPLIT (operand_dtype 2, "fp16x3"): every MMA operand is carried as an fp16 head plus the fp16 tail of its rounding
 // error and every product as head*head + tail*head + head*tail (fp32 accumulate): ~22-bit operands, the parity mode that
-// meets the 1e-4 rendered-RGB contract.  The tails take the TMEM / shared-memory / scratch space of tile group 1, so a CTA
-// then keeps ONE tile in flight (group 1's warps idle): activations tails in columns [384, 512), embedding tails in group
-// 1's arena chunks, N-half 0 of a wide layer is staged in columns [128, 256) instead of registers.
+// meets the 1e-4 rendered-RGB contract.  The tails take the TMEM / shared-memory space of tile group 1, so a CTA then
+// keeps ONE tile in flight: activation tails in columns [384, 512), embedding tails in group 1's arena chunks.  Both
+// groups' warps work on that tile: warps q and 4+q read the same TMEM lane quadrant and split every epilogue's 32-column
+// blocks (group g takes the blocks [g * nb / 2, (g + 1) * nb / 2) of each N-half), so every c2m barrier counts 8 warps.
+// Per-row scalar work (sample placement, skinning blend, embedding, heads, per-sample outputs) stays on group 0.
+// Columns [128, 256) are the accumulator of a wide layer's N-half 1, whose MMAs then overlap the epilogue of half 0.
 // SAVE (training forward, b200r_field_fwd with a tape): every epilogue also records the 16-bit operand it produced in the
 // tape's chunk image and one word of ReLU sign bits per 32 columns (program.h TapeLayout) for the backward kernels.
 template <class Op, int B, int LMAX, bool DENSE, int WIDTH, bool SPLIT, bool SAVE>
@@ -118,20 +123,14 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
   uint64_t* c2m = bars + 3 * kNumStages;      // [group][4] compute warps -> MMA thread, indexed by BAR_*
   uint64_t* m2c = bars + 3 * kNumStages + 8;  // [group][4] MMA thread (tcgen05.commit) -> compute warps
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3 * kNumStages + 16);
-  // SPLIT + SAVE: tile group 1's warps are idle (their resources hold the operand tails) and act as TAPE WRITERS: group 0 posts
-  // (tile, chunk, first activation column, columns) after an epilogue has put its 16-bit heads into TMEM; the writers read
-  // them back (tcgen05.ld, same lane quadrants) and do the global stores, off the critical path of the one tile in flight.
-  uint64_t* act_ready = bars + 3 * kNumStages + 17;  // group 0 (4 warps) -> writers: command posted, activations complete
-  uint64_t* act_free = act_ready + 1;                // writers (4 warps) -> group 0: activations read, columns may be overwritten
-  volatile int32_t* proxy_cmd = reinterpret_cast<volatile int32_t*>(act_free + 1);  // [4]
-  constexpr bool kProxy = SPLIT && SAVE;
+  // SPLIT: MODE 1 partial sdf dot products, [2 * (WIDTH / 64) blocks][128 rows], summed by group 0 in block order
+  const uint32_t sdf_part_s = smem_u32(bars) + kBarBytes;
 
   const int warp = __shfl_sync(0xffffffffu, threadIdx.x >> 5, 0), lane = threadIdx.x & 31;  // warp-uniform for the compiler
   if (threadIdx.x == 0) {
     for (int i = 0; i < kNumStages; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&full_bar[kNumStages + i], 1); mbar_init(&empty_bar[i], kCluster); }
-    for (int i = 0; i < 8; ++i) { mbar_init(&c2m[i], 4); mbar_init(&m2c[i], 1); }  // one arrival per warp of the group
-    mbar_init(act_ready, 4);
-    mbar_init(act_free, 4);
+    // one arrival per warp working on the group's tile (SPLIT: both groups' warps)
+    for (int i = 0; i < 8; ++i) { mbar_init(&c2m[i], SPLIT ? 8 : 4); mbar_init(&m2c[i], 1); }
     fence_barrier_init();
   }
   if (warp == 9) tmem_alloc(tmem_slot, kTmemCols);
@@ -220,7 +219,10 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
         const uint32_t tile2 = n << 3;  // descriptor offset of a slot's second weight tile (n rows x 128 B)
         if (g == 1) skip(cnt);
         const uint32_t wt = Bk.wait, cm = Bk.commit;
-        if (wt) {
+        // SPLIT: N-half 1 of a wide layer (the block that waits on BAR_H0) accumulates into columns [128, 256), so it
+        // need not wait for the epilogue to drain half 0
+        const bool half1 = SPLIT && wt == BAR_H0;
+        if (wt && !half1) {
           mbar_wait(&c2m_g[wt], (bar_phase >> wt) & 1u);
           bar_phase ^= 1u << wt;
         }
@@ -228,6 +230,7 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
         if constexpr (SPLIT) {
           // one ring slot per K chunk: [head tile][tail tile]; operand tails: embedding chunks of group 1's arena,
           // activation columns + kTmemGroup.  D += Ah Wh + Al Wh + Ah Wl per k-step.
+          const uint32_t dd = half1 ? d + kTmemGroup : d;
           const uint32_t ks_ss[2] = {ss & 7u, (ss >> 3) & 7u};
           const uint32_t n_ss = ss ? (ks_ss[1] ? 2u : 1u) : 0u;
           for (uint32_t c = 0; c < n_ss; ++c) {
@@ -237,9 +240,9 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
             if (elect_one()) {
               const uint32_t ah = ad_lo0 + (uint32_t)((Bk.ss_chunks >> (4 * c)) & 15) * (kAChunkBytes >> 4), al = ah + (kArenaGroup >> 4);
               for (uint32_t k = 0; k < ks_ss[c]; ++k) {
-                umma_f16_ss(d, mk(ah + 2 * k), mk(bd + 2 * k), idesc, acc | k);
-                umma_f16_ss(d, mk(al + 2 * k), mk(bd + 2 * k), idesc, 1u);
-                umma_f16_ss(d, mk(ah + 2 * k), mk(bl + 2 * k), idesc, 1u);
+                umma_f16_ss(dd, mk(ah + 2 * k), mk(bd + 2 * k), idesc, acc | k);
+                umma_f16_ss(dd, mk(al + 2 * k), mk(bd + 2 * k), idesc, 1u);
+                umma_f16_ss(dd, mk(ah + 2 * k), mk(bl + 2 * k), idesc, 1u);
               }
               release();
               if (last && cm) umma_commit(&m2c_g[cm]);
@@ -257,9 +260,9 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
             const uint32_t ks = last ? (uint32_t)Bk.ts_ks2_last : 4u;
             if (elect_one()) {
               for (uint32_t k = 0; k < ks; ++k) {
-                umma_f16_ts(d, a + 8 * k, mk(bd + 2 * k), idesc, acc | k);
-                umma_f16_ts(d, a + kTmemGroup + 8 * k, mk(bd + 2 * k), idesc, 1u);
-                umma_f16_ts(d, a + 8 * k, mk(bl + 2 * k), idesc, 1u);
+                umma_f16_ts(dd, a + 8 * k, mk(bd + 2 * k), idesc, acc | k);
+                umma_f16_ts(dd, a + kTmemGroup + 8 * k, mk(bd + 2 * k), idesc, 1u);
+                umma_f16_ts(dd, a + 8 * k, mk(bl + 2 * k), idesc, 1u);
               }
               release();
               if (last && cm) umma_commit(&m2c_g[cm]);
@@ -322,27 +325,32 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
     // =============================================================== compute / epilogue warps
     asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(kRegsCompute));
     const int g = warp >> 2, q = warp & 3;
+    // SPLIT: both groups work on group 0's tile (its TMEM, arena, frame block, scratch and barriers); group g then only
+    // selects the column blocks of an epilogue, and group 0 alone does the per-row scalar work (`lead`)
+    const int tg = SPLIT ? 0 : g;
+    const bool lead = !SPLIT || g == 0;
+    constexpr int kTileThreads = SPLIT ? kComputeThreads : kGroupThreads;  // threads working on one tile
     const int gtid = threadIdx.x & (kGroupThreads - 1);
+    const int ttid = SPLIT ? (int)threadIdx.x : gtid;
     const uint32_t row = (uint32_t)(q * 32 + lane);  // tile row == TMEM lane
     const uint32_t t_lane = tmem_base + ((uint32_t)(q * 32) << 16);
-    const uint32_t tD = t_lane + kTmemAcc + kTmemGroup * g;  // this group's accumulator
-    const uint32_t tA = t_lane + kTmemAct + kTmemGroup * g;  // this group's 16-bit activations (2 per column)
-    constexpr uint32_t kTail = kTmemGroup;                     // SPLIT: activation tails live in group 1's columns
-    const uint32_t tS = t_lane + kTmemAcc + kTmemGroup;        // SPLIT: staging of a wide layer's N-half 0 (group 1's accumulator)
-    uint64_t* c2m_g = c2m + 4 * g;
-    uint64_t* m2c_g = m2c + 4 * g;
+    const uint32_t tD = t_lane + kTmemAcc + kTmemGroup * tg;  // this tile's accumulator
+    const uint32_t tA = t_lane + kTmemAct + kTmemGroup * tg;  // this tile's 16-bit activations (2 per column)
+    constexpr uint32_t kTail = kTmemGroup;                      // SPLIT: activation tails live in group 1's columns
+    uint64_t* c2m_g = c2m + 4 * tg;
+    uint64_t* m2c_g = m2c + 4 * tg;
     uint32_t all_phase = 0, half_phase = 0;
     constexpr int HN = WIDTH / 2, NBLK = HN / 32;  // N-half of the wide layers; 32-column blocks per half
     const int lid_delta = 0, lid_vis = B > 0 ? 3 : 0, lid_base = lid_vis + 2, lid_rgb0 = lid_base + p.desc.D + 1,
               lid_color = lid_rgb0 + 1, lid_feat = lid_color + 3, lid_dense = lid_feat + (p.desc.has_feature ? 6 : 0);
     const ConstLayout& CL = P.cl;
     const FrameLayout& FL = P.fl;
-    float* fblk_g = fblk + g * FL.n_floats;
+    float* fblk_g = fblk + tg * FL.n_floats;
     const uint32_t cblk_s = smem_u32(cblk), fblk_s = smem_u32(fblk_g);
-    const uint32_t pe_s = smem_u32(arena) + g * kArenaGroup, extra_s = pe_s + kAChunkBytes;
+    const uint32_t pe_s = smem_u32(arena) + tg * kArenaGroup, extra_s = pe_s + kAChunkBytes;
     const uint32_t rowx = row * 128u + ((row & 7u) << 4);  // 16-B group gq of this row lives at chunk + (rowx ^ (gq << 4))
     const uint32_t sc_s = cblk_s + 4u * CL.scalars;
-    uint4* scr = p.scratch + ((size_t)blockIdx.x * kGroups + g) * (kTileRows * 32) + row;  // [32 uint4][128 rows]
+    uint4* scr = p.scratch + ((size_t)blockIdx.x * kGroups + tg) * (kTileRows * 32) + row;  // [32 uint4][128 rows]
     uint4* scr_t = scr + kTileRows * 32;                                                  // SPLIT: tails (group 1's scratch)
     // ---- training tape (SAVE): this row's slice of the current tile's chunk images / sign words
     const TapeLayout& TL = p.tape;
@@ -354,32 +362,6 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
       if constexpr (SAVE) {
         if (tape_tile != nullptr && chunk >= 0) {
           chunk_st32(tape_tile + tape_row_off(TL.n_a, chunk + (col0 >> 6), row), row, (uint32_t)(col0 & 63) >> 3, o);
-        }
-      }
-    };
-    // ---- tape-writer proxy (kProxy): group 0 side
-    uint32_t proxy_phase = 0;
-    bool proxy_pending = false;
-    int cur_tile = 0;
-    // activations [tcol, tcol + ncols) (TMEM columns of packed pairs, ncols a multiple of 16) are complete: hand them over
-    auto proxy_save = [&](int chunk, int tcol, int ncols) {
-      if constexpr (kProxy) {
-        if (tape_tile == nullptr || chunk < 0) return;
-        tc_fence_before_sync();
-        if (gtid == 0) { proxy_cmd[0] = cur_tile; proxy_cmd[1] = chunk; proxy_cmd[2] = tcol; proxy_cmd[3] = ncols; }
-        __syncwarp();
-        if (lane == 0) mbar_arrive(act_ready);
-        proxy_pending = true;
-      }
-    };
-    // before anything overwrites the activation columns: the writers must have read the last hand-over
-    auto proxy_wait = [&]() {
-      if constexpr (kProxy) {
-        if (proxy_pending) {
-          mbar_wait(act_free, proxy_phase);
-          proxy_phase ^= 1;
-          tc_fence_after_sync();
-          proxy_pending = false;
         }
       }
     };
@@ -458,9 +440,9 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
     };
     // finished GEMM of n (<= 128) columns: relu(acc + bias) -> activations [0, n)
     auto epi_relu_act = [&](uint32_t bias, int n, int save_chunk, int mask_slot) {
-      proxy_wait();
+      const int nb = n >> 5;
 #pragma unroll 1
-      for (int blk = 0; blk < (n >> 5); ++blk) {
+      for (int blk = SPLIT ? (g * nb) >> 1 : 0; blk < (SPLIT ? ((g + 1) * nb) >> 1 : nb); ++blk) {
         uint32_t ra[32], o[16], ot[SPLIT ? 16 : 1];
         tmem_ld32_issue(tD + 32 * blk, ra);
         tmem_ld_wait32(ra);
@@ -471,11 +453,10 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
           relu_pack32(ra, bias + 128u * blk, o, o);
         }
         tmem_st16(tA + 16 * blk, o);
-        if constexpr (!kProxy) tape_st32(save_chunk, 32 * blk, o);
+        tape_st32(save_chunk, 32 * blk, o);
         mask_st(mask_slot, blk, sign_word());
       }
       tmem_st_wait();
-      proxy_save(save_chunk, 0, n >> 1);
     };
     // One 2*hn-wide layer issued as two N-halves on this group's accumulator (program.h pipe5).
     //   MODE 0: relu(acc + bias) -> activations (in place: half 0 is held in registers until the layer's MMAs are done)
@@ -484,8 +465,6 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
     float sdf_acc = 0.f;
     auto chain_layer = [&](auto mode_tag, uint32_t bias, int save_chunk, int mask_slot) {
       constexpr int MODE = decltype(mode_tag)::value;
-      uint32_t hold[SPLIT ? 1 : NBLK][16];
-      uint32_t mwords[SAVE ? 2 * NBLK : 1];
       auto math = [&](const uint32_t (&ra)[32], int col0, uint32_t (&o)[16], uint32_t (&ot)[16]) {  // col0: first feature of these 32 columns
         const uint32_t ba = bias + 4u * (uint32_t)col0;
         if (MODE == 0) {
@@ -506,7 +485,8 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
             pack_ht(y0, y1, o[2 * g4], ot[2 * g4]);
             pack_ht(y2, y3, o[2 * g4 + 1], ot[2 * g4 + 1]);
           }
-          sdf_acc += s0 + s1;
+          if constexpr (SPLIT) sts32(sdf_part_s + 4u * ((uint32_t)(col0 >> 5) * kTileRows + row), s0 + s1);  // summed in block order
+          else sdf_acc += s0 + s1;
 #pragma unroll
           for (int j = 0; j < 4; ++j) {
             scr[(size_t)((col0 >> 3) + j) * kTileRows] = make_uint4(o[4 * j], o[4 * j + 1], o[4 * j + 2], o[4 * j + 3]);
@@ -537,86 +517,118 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
           }
         }
       };
-      // ---- N-half 0: drain the accumulator so the MMAs of half 1 can start
-      wait_half(0);
+      if constexpr (SPLIT) {
+        // Group g takes the BPG blocks [g * BPG, (g + 1) * BPG) of each N-half.  Half 1 accumulates in columns [128, 256),
+        // so its MMAs run while half 0 is drained; half 0's heads and tails wait in registers until the layer's MMAs have
+        // read its input.
+        constexpr int BPG = NBLK / 2;
+        const int blk0 = g * BPG;
+        uint32_t hd[BPG][16], tl[BPG][16];
+        uint32_t mw[SAVE ? 2 * BPG : 1];
+        wait_half(0);
 #pragma unroll
-      for (int bp = 0; bp < NBLK; bp += 2) {  // two 32-column blocks per TMEM round trip
-        uint32_t rp[2][32];
-        tmem_ld32_issue(tD + 32 * bp, rp[0]);
-        tmem_ld32_issue(tD + 32 * (bp + 1), rp[1]);
-        tmem_ld_wait32(rp[0]);
-        tmem_ld_wait32(rp[1]);
+        for (int i = 0; i < BPG; ++i) {  // one block per TMEM round trip: keeps half 0's heads and tails in registers without spills
+          uint32_t ra[32];
+          tmem_ld32_issue(tD + 32 * (blk0 + i), ra);
+          tmem_ld_wait32(ra);
+          math(ra, 32 * (blk0 + i), hd[i], tl[i]);
+          tape_st32(save_chunk, 32 * (blk0 + i), hd[i]);
+          if constexpr (SAVE) mw[i] = sign_word();
+        }
+        // ---- N-half 1: the layer's input has been read, activations can be overwritten
+        wait_half(1);
+        if (MODE != 1) {
 #pragma unroll
-        for (int h2 = 0; h2 < 2; ++h2) {
-          const int blk = bp + h2;
-          if constexpr (SPLIT) {
-            uint32_t o[16], ot[16];
-            math(rp[h2], 32 * blk, o, ot);
-            if (MODE != 1) { tmem_st16(tS + 16 * blk, o); tmem_st16(tS + 64 + 16 * blk, ot); }
-            if (!kProxy || MODE == 1) tape_st32(save_chunk, 32 * blk, o);
-          } else {
+          for (int i = 0; i < BPG; ++i) {
+            tmem_st16(tA + 16 * (blk0 + i), hd[i]);
+            tmem_st16(tA + kTail + 16 * (blk0 + i), tl[i]);
+          }
+        }
+#pragma unroll
+        for (int i = 0; i < BPG; ++i) {  // one block per round trip too: the other group's warp covers the latency
+          const int blk = blk0 + i;
+          uint32_t ra[32], o[16], ot[16];
+          tmem_ld32_issue(tD + kTmemGroup + 32 * blk, ra);
+          tmem_ld_wait32(ra);
+          math(ra, HN + 32 * blk, o, ot);
+          if (MODE != 1) {
+            tmem_st16(tA + (HN >> 1) + 16 * blk, o);
+            tmem_st16(tA + kTail + (HN >> 1) + 16 * blk, ot);
+          }
+          tape_st32(save_chunk, HN + 32 * blk, o);
+          if constexpr (SAVE) mw[BPG + i] = sign_word();
+        }
+        if constexpr (SAVE) {  // this group's sign words of each half: words [blk0, blk0 + BPG) and NBLK further
+          if (mask_row != nullptr && mask_slot >= 0) {
+            uint32_t* mp = mask_row + (size_t)mask_slot * (kTileRows * kMaskWords);
+            if constexpr (BPG == 2) {
+              *reinterpret_cast<uint2*>(mp + blk0) = make_uint2(mw[0], mw[1]);
+              *reinterpret_cast<uint2*>(mp + NBLK + blk0) = make_uint2(mw[2], mw[3]);
+            } else {
+#pragma unroll
+              for (int i = 0; i < BPG; ++i) { mp[blk0 + i] = mw[i]; mp[NBLK + blk0 + i] = mw[BPG + i]; }
+            }
+          }
+        }
+        if (MODE != 1) tmem_st_wait();
+        tc_fence_before_sync();
+        warp_arrive(&c2m_g[BAR_H1]);
+      } else {
+        // ---- N-half 0: drain the accumulator so the MMAs of half 1 can start
+        uint32_t hold[NBLK][16];
+        uint32_t mwords[SAVE ? 2 * NBLK : 1];
+        wait_half(0);
+#pragma unroll
+        for (int bp = 0; bp < NBLK; bp += 2) {  // two 32-column blocks per TMEM round trip
+          uint32_t rp[2][32];
+          tmem_ld32_issue(tD + 32 * bp, rp[0]);
+          tmem_ld32_issue(tD + 32 * (bp + 1), rp[1]);
+          tmem_ld_wait32(rp[0]);
+          tmem_ld_wait32(rp[1]);
+#pragma unroll
+          for (int h2 = 0; h2 < 2; ++h2) {
+            const int blk = bp + h2;
             math(rp[h2], 32 * blk, hold[blk], hold[blk]);
             tape_st32(save_chunk, 32 * blk, hold[blk]);
+            if constexpr (SAVE) mwords[blk] = sign_word();
           }
-          if constexpr (SAVE) mwords[blk] = sign_word();
         }
-      }
-      if (SPLIT && MODE != 1) tmem_st_wait();
-      tc_fence_before_sync();
-      warp_arrive(&c2m_g[BAR_H0]);
-      // ---- N-half 1: the layer's input has been read, activations can be overwritten
-      wait_half(1);
-      if (MODE != 1) proxy_wait();
-      if (MODE != 1) {
-        if constexpr (SPLIT) {  // staged heads and tails -> activation buffers, NBLK blocks per TMEM round trip
-#pragma unroll
-          for (int part = 0; part < 2; ++part) {
-            uint32_t t[NBLK][16];
-#pragma unroll
-            for (int blk = 0; blk < NBLK; ++blk) tmem_ld16u_issue(tS + 64 * part + 16 * blk, t[blk]);
-#pragma unroll
-            for (int blk = 0; blk < NBLK; ++blk) tmem_ld_wait16(t[blk]);
-#pragma unroll
-            for (int blk = 0; blk < NBLK; ++blk) tmem_st16(tA + (part ? kTail : 0u) + 16 * blk, t[blk]);
-          }
-        } else {
+        tc_fence_before_sync();
+        warp_arrive(&c2m_g[BAR_H0]);
+        // ---- N-half 1: the layer's input has been read, activations can be overwritten
+        wait_half(1);
+        if (MODE != 1) {
 #pragma unroll
           for (int blk = 0; blk < NBLK; ++blk) tmem_st16(tA + 16 * blk, hold[blk]);
         }
-      }
 #pragma unroll
-      for (int bp = 0; bp < NBLK; bp += 2) {
-        uint32_t rp[2][32];
-        tmem_ld32_issue(tD + 32 * bp, rp[0]);
-        tmem_ld32_issue(tD + 32 * (bp + 1), rp[1]);
-        tmem_ld_wait32(rp[0]);
-        tmem_ld_wait32(rp[1]);
+        for (int bp = 0; bp < NBLK; bp += 2) {
+          uint32_t rp[2][32];
+          tmem_ld32_issue(tD + 32 * bp, rp[0]);
+          tmem_ld32_issue(tD + 32 * (bp + 1), rp[1]);
+          tmem_ld_wait32(rp[0]);
+          tmem_ld_wait32(rp[1]);
 #pragma unroll
-        for (int h2 = 0; h2 < 2; ++h2) {
-          const int blk = bp + h2;
-          uint32_t o[16], ot[SPLIT ? 16 : 1];
-          if constexpr (SPLIT) {
-            math(rp[h2], HN + 32 * blk, o, ot);
-            if (MODE != 1) tmem_st16(tA + kTail + (HN >> 1) + 16 * blk, ot);
-          } else {
+          for (int h2 = 0; h2 < 2; ++h2) {
+            const int blk = bp + h2;
+            uint32_t o[16];
             math(rp[h2], HN + 32 * blk, o, o);
+            if (MODE != 1) tmem_st16(tA + (HN >> 1) + 16 * blk, o);
+            tape_st32(save_chunk, HN + 32 * blk, o);
+            if constexpr (SAVE) mwords[NBLK + blk] = sign_word();
           }
-          if (MODE != 1) tmem_st16(tA + (HN >> 1) + 16 * blk, o);
-          if (!kProxy || MODE == 1) tape_st32(save_chunk, HN + 32 * blk, o);
-          if constexpr (SAVE) mwords[NBLK + blk] = sign_word();
         }
-      }
-      if constexpr (SAVE) {  // the layer's sign words in one (or two) 16-B stores
-        if (mask_row != nullptr && mask_slot >= 0) {
-          uint4* mp = reinterpret_cast<uint4*>(mask_row + (size_t)mask_slot * (kTileRows * kMaskWords));
-          mp[0] = make_uint4(mwords[0], mwords[1], mwords[2], mwords[3]);
-          if (NBLK > 2) mp[1] = make_uint4(mwords[4 % (2 * NBLK)], mwords[5 % (2 * NBLK)], mwords[6 % (2 * NBLK)], mwords[7 % (2 * NBLK)]);
+        if constexpr (SAVE) {  // the layer's sign words in one (or two) 16-B stores
+          if (mask_row != nullptr && mask_slot >= 0) {
+            uint4* mp = reinterpret_cast<uint4*>(mask_row + (size_t)mask_slot * (kTileRows * kMaskWords));
+            mp[0] = make_uint4(mwords[0], mwords[1], mwords[2], mwords[3]);
+            if (NBLK > 2) mp[1] = make_uint4(mwords[4 % (2 * NBLK)], mwords[5 % (2 * NBLK)], mwords[6 % (2 * NBLK)], mwords[7 % (2 * NBLK)]);
+          }
         }
+        if (MODE != 1) tmem_st_wait();
+        tc_fence_before_sync();
+        warp_arrive(&c2m_g[BAR_H1]);
       }
-      if (MODE != 1) tmem_st_wait();
-      tc_fence_before_sync();
-      warp_arrive(&c2m_g[BAR_H1]);
-      if (MODE != 1) proxy_save(save_chunk, 0, HN);
     };
 
     // 16-bit element `c` (0..63) of this row in an operand chunk
@@ -668,77 +680,55 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
       }
     };
     auto dense_warp = [&](const float3& x, uint32_t bias1, int lid0, int w) -> float3 {
-      embed(x, 6);
-      put16(pe_s, 39, 0.f);  // 39 embedding columns; the third k-step reads up to column 47
-      sts128(pe_s + (rowx ^ (5u << 4)), make_uint4(0u, 0u, 0u, 0u));
-      if constexpr (SPLIT) sts128(pe_s + kArenaGroup + (rowx ^ (5u << 4)), make_uint4(0u, 0u, 0u, 0u));
-      tape_copy_row(TL.a_dpe[w], pe_s, 6);
+      if (lead) {
+        embed(x, 6);
+        put16(pe_s, 39, 0.f);  // 39 embedding columns; the third k-step reads up to column 47
+        sts128(pe_s + (rowx ^ (5u << 4)), make_uint4(0u, 0u, 0u, 0u));
+        if constexpr (SPLIT) sts128(pe_s + kArenaGroup + (rowx ^ (5u << 4)), make_uint4(0u, 0u, 0u, 0u));
+        tape_copy_row(TL.a_dpe[w], pe_s, 6);
+      }
       arrive_all();
 #pragma unroll 1
       for (int l = 0; l < 2; ++l)
         chain_layer(IC<0>{}, l == 0 ? bias1 : bias_s(lid0 + 1), l == 0 ? TL.a_dh1[w] : TL.a_dh2[w], l == 0 ? TL.m_dh1[w] : TL.m_dh2[w]);
       wait_all();
+      if (!lead) return x;
       float m[16];
       tmem_ld16(tD, m);
       const uint32_t b3 = bias_s(lid0 + 2);
       return make_float3(x.x + 0.1f * (m[0] + lds32(b3)), x.y + 0.1f * (m[1] + lds32(b3 + 4)), x.z + 0.1f * (m[2] + lds32(b3 + 8)));
     };
 
-    if constexpr (kProxy) {
-      if (g == 1) {  // ================================================= tape writers (see act_ready above)
-        uint32_t ph = 0;
-        for (;;) {
-          mbar_wait(act_ready, ph);
-          ph ^= 1;
-          tc_fence_after_sync();
-          const int c_tile = proxy_cmd[0], c_chunk = proxy_cmd[1], c_col = proxy_cmd[2], c_n = proxy_cmd[3];
-          if (c_chunk < 0) break;  // group 0 is done
-          uint32_t regs[8][16];
-          const int nblk = c_n >> 4;  // 16 columns = 32 values = one 64-B block of the row
-#pragma unroll
-          for (int b8 = 0; b8 < 8; ++b8)
-            if (b8 < nblk) tmem_ld16u(t_lane + kTmemAct + (uint32_t)c_col + 16u * b8, regs[b8]);
-          tc_fence_before_sync();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(act_free);
-          uint8_t* tt = p.tape_a + (size_t)c_tile * TL.n_a * kChunkBytes;
-#pragma unroll
-          for (int b8 = 0; b8 < 8; ++b8)
-            if (b8 < nblk) chunk_st32(tt + tape_row_off(TL.n_a, c_chunk + (b8 >> 1), row), row, (uint32_t)(b8 & 1) * 4u, regs[b8]);
-        }
-      }
-    }
-    for (int it = 0; it < (SPLIT && g == 1 ? 0 : iters); ++it) {  // SPLIT: group 1's resources hold the operand tails
-      const int tile_raw = (kActive * it + g) * (int)gridDim.x + (int)blockIdx.x;
+    for (int it = 0; it < iters; ++it) {
+      const int tile_raw = (kActive * it + tg) * (int)gridDim.x + (int)blockIdx.x;
       const bool dead_tile = tile_raw >= p.n_tiles;
       const int tile = dead_tile ? p.n_tiles - 1 : tile_raw;
       const int f = tile / p.tiles_per_frame;
       const int r_raw = (tile - f * p.tiles_per_frame) * kTileRows + (int)row;
-      const bool live = !dead_tile && r_raw < p.ND;
+      const bool live = lead && !dead_tile && r_raw < p.ND;  // this thread writes the row's per-sample outputs
       const int r_in = r_raw < p.ND ? r_raw : p.ND - 1;
       const int n = r_in / p.rays.D;
       const int k = r_in - n * p.rays.D;
       const size_t s = (size_t)f * p.ND + r_in;
-      cur_tile = tile;
       if constexpr (SAVE) {
         tape_tile = dead_tile ? nullptr : p.tape_a + (size_t)tile * TL.n_a * kChunkBytes;
         mask_row = dead_tile ? nullptr : p.tape_mask + ((size_t)tile * TL.n_mask * kTileRows + row) * kMaskWords;
       }
 
       // ------------------------------------------------ stage this frame's block in shared memory
-      named_bar_sync(1 + g, kGroupThreads);  // the group is done with the previous block
+      named_bar_sync(1 + tg, kTileThreads);  // the tile's warps are done with the previous block
       {
         const float4* src = reinterpret_cast<const float4*>(p.workspace + CL.n_floats + (size_t)f * FL.n_floats);
         float4* dst = reinterpret_cast<float4*>(fblk_g);
-        for (int i = gtid; i < FL.n_floats / 4; i += kGroupThreads) dst[i] = __ldg(src + i);
+        for (int i = ttid; i < FL.n_floats / 4; i += kTileThreads) dst[i] = __ldg(src + i);
       }
-      named_bar_sync(1 + g, kGroupThreads);
+      named_bar_sync(1 + tg, kTileThreads);
 
       // ------------------------------------------------ sample placement (sample_cam_rays)
       const bool pts = p.points != nullptr;  // b200r_points_fwd: canonical points are given, only NeRF.forward runs
       float h0 = 0.f, h1 = 0.f, depth = 0.f, delta = 0.f;
       float3 xyz_cam = make_float3(0.f, 0.f, 0.f), xyz_t = xyz_cam, dir_f = xyz_cam;
-      if (!pts) {
+      if (lead && !pts) {
         const float* hx = p.rays.hxy + ((size_t)f * p.rays.N + n) * 3;
         h0 = __ldg(hx); h1 = __ldg(hx + 1);
         const float h2 = __ldg(hx + 2);
@@ -769,7 +759,7 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
         xyz_t = qrot(qi, xyz_cam);
         xyz_t.x += ti.x; xyz_t.y += ti.y; xyz_t.z += ti.z;
         dir_f = qrot(qi, dir_cam);
-      } else {
+      } else if (lead) {
         const float* px = p.points + s * 3;
         xyz_t = make_float3(__ldg(px), __ldg(px + 1), __ldg(px + 2));
         if (p.point_dirs) {
@@ -785,7 +775,7 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
       constexpr int NP = B > 0 ? (3 * B + 15) / 16 * 8 : 1;  // packed pairs of the zero-padded bone-coordinate row
       auto skin_warp = [&](const float3& x, uint32_t binv, uint32_t se3, uint32_t bias1, float& entropy, float& delta_skin, int w) -> float3 {
         float dist2[B > 0 ? B : 1];
-        {
+        if (lead) {
           uint32_t u[NP], ut[SPLIT ? NP : 1];
 #pragma unroll
           for (int i = 0; i < NP; ++i) u[i] = 0u;
@@ -814,7 +804,6 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
             pack_ht(v[2], v[3], u[3 * b2 + 1], ut[SPLIT ? 3 * b2 + 1 : 0]);
             pack_ht(v[4], v[5], u[3 * b2 + 2], ut[SPLIT ? 3 * b2 + 2 : 0]);
           }
-          proxy_wait();
           tmem_st32(tA, u);
           if (NP > 32) tmem_st8(tA + 32, u + (NP > 32 ? 32 : 0));
           if constexpr (SPLIT) {
@@ -838,6 +827,7 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
         gemm();
         epi_relu_act(bias_s(lid_delta + 1), 64, TL.a_h2[w], TL.m_h2[w]);
         gemm();
+        if (!lead) return x;
         float dl[32];
         tmem_ld32(tD, dl);
         const uint32_t b3 = bias_s(lid_delta + 2);
@@ -943,9 +933,9 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
       // ------------------------------------------------ outputs that are final before the MLPs run
       auto st3 = [&](float* dst, float a, float b, float c) { if (dst && live) { dst[s * 3] = a; dst[s * 3 + 1] = b; dst[s * 3 + 2] = c; } };
       auto st1 = [&](float* dst, float a) { if (dst && live) dst[s] = a; };
-      if (pts) {
+      if (lead && pts) {
         st3(p.out.xyz, xyz.x, xyz.y, xyz.z);
-      } else {
+      } else if (lead) {
         // field_to_cam with the partner frame's camera, pinhole projection, flow (nerf.py:948-997)
         const float* cn = fblk_g + FL.cam_partner;
         const Q4 qn = {cn[11], cn[12], cn[13], cn[14]};
@@ -983,26 +973,28 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
       }
 
       // ------------------------------------------------ positional embedding of the canonical point
-      embed(xyz, LMAX);
-      sts16(pe_s + (rowx ^ (7u << 4)) + 14u, (uint16_t)0);  // zero pad column 63 of CH_PE
-      if constexpr (SPLIT) sts16(pe_s + kArenaGroup + (rowx ^ (7u << 4)) + 14u, (uint16_t)0);
-      if (LMAX > 10) {  // CH_EXTRA holds 12 values (columns 63..74); its k-step reads 16 columns
-        sts32(extra_s + (rowx ^ (1u << 4)) + 8u, 0.f);
-        sts32(extra_s + (rowx ^ (1u << 4)) + 12u, 0.f);
-        if constexpr (SPLIT) {
-          sts32(extra_s + kArenaGroup + (rowx ^ (1u << 4)) + 8u, 0.f);
-          sts32(extra_s + kArenaGroup + (rowx ^ (1u << 4)) + 12u, 0.f);
+      if (lead) {
+        embed(xyz, LMAX);
+        sts16(pe_s + (rowx ^ (7u << 4)) + 14u, (uint16_t)0);  // zero pad column 63 of CH_PE
+        if constexpr (SPLIT) sts16(pe_s + kArenaGroup + (rowx ^ (7u << 4)) + 14u, (uint16_t)0);
+        if (LMAX > 10) {  // CH_EXTRA holds 12 values (columns 63..74); its k-step reads 16 columns
+          sts32(extra_s + (rowx ^ (1u << 4)) + 8u, 0.f);
+          sts32(extra_s + (rowx ^ (1u << 4)) + 12u, 0.f);
+          if constexpr (SPLIT) {
+            sts32(extra_s + kArenaGroup + (rowx ^ (1u << 4)) + 8u, 0.f);
+            sts32(extra_s + kArenaGroup + (rowx ^ (1u << 4)) + 12u, 0.f);
+          }
         }
-      }
 
-      tape_copy_row(TL.a_pe, pe_s, 8);
-      if (LMAX > 10) tape_copy_row(TL.a_extra, extra_s, 2);
+        tape_copy_row(TL.a_pe, pe_s, 8);
+        if (LMAX > 10) tape_copy_row(TL.a_extra, extra_s, 2);
+      }
       // ------------------------------------------------ visibility MLP (VisField.forward)
       if (!pts) {
       gemm();
       epi_relu_act(bias_s(lid_vis), 64, TL.a_vis[0], TL.m_vis[0]);
       gemm();
-      {
+      if (lead) {
         const uint32_t b2 = bias_s(lid_vis + 1), vw = cblk_s + 4u * CL.vis_w;
         float a0 = 0.f, a1 = 0.f;
 #pragma unroll 1
@@ -1040,18 +1032,20 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
           epi_relu_act(bias_s(lid_feat + i), 128, TL.a_feat[i], TL.m_feat[i]);
         }
         gemm();
-        float v16[16];
-        tmem_ld16(tD, v16);
-        const uint32_t bf = bias_s(lid_feat + 5);
-        float nn = 0.f;
+        if (lead) {
+          float v16[16];
+          tmem_ld16(tD, v16);
+          const uint32_t bf = bias_s(lid_feat + 5);
+          float nn = 0.f;
 #pragma unroll
-        for (int j = 0; j < 16; ++j) { v16[j] += lds32(bf + 4u * j); nn += v16[j] * v16[j]; }
-        const float inv = rsqrtf(nn);
-        if (p.out.feat_norm && live) p.out.feat_norm[s] = inv;
-        if (p.out.feature && live) {
-          float4* fo = reinterpret_cast<float4*>(p.out.feature + s * 16);
+          for (int j = 0; j < 16; ++j) { v16[j] += lds32(bf + 4u * j); nn += v16[j] * v16[j]; }
+          const float inv = rsqrtf(nn);
+          if (p.out.feat_norm && live) p.out.feat_norm[s] = inv;
+          if (p.out.feature && live) {
+            float4* fo = reinterpret_cast<float4*>(p.out.feature + s * 16);
 #pragma unroll
-          for (int j = 0; j < 4; ++j) fo[j] = make_float4(v16[4 * j] * inv, v16[4 * j + 1] * inv, v16[4 * j + 2] * inv, v16[4 * j + 3] * inv);
+            for (int j = 0; j < 4; ++j) fo[j] = make_float4(v16[4 * j] * inv, v16[4 * j + 1] * inv, v16[4 * j + 2] * inv, v16[4 * j + 3] * inv);
+          }
         }
       }
 
@@ -1061,6 +1055,15 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
 #pragma unroll 1
       for (int j = 0; j < p.desc.D; ++j) chain_layer(IC<0>{}, bias_s(lid_base + j), TL.a_base[j], TL.m_base[j]);
       chain_layer(IC<1>{}, bias_s(lid_base + p.desc.D), TL.a_base[p.desc.D], TL.m_base[p.desc.D]);
+      if constexpr (SPLIT) {  // both groups' partial dot products, summed in block order (as the one-group order)
+        if (lead) {
+          named_bar_sync(4 + q, 64);  // warps q and 4 + q
+#pragma unroll
+          for (int blk = 0; blk < 2 * NBLK; ++blk) sdf_acc += lds32(sdf_part_s + 4u * ((uint32_t)blk * kTileRows + row));
+        } else {
+          named_bar_arrive(4 + q, 64);
+        }
+      }
       const float sdf = sdf_acc + lds32(sc_s + 4u * SC_SDF_B);
       const float ibeta = lds32(sc_s + 4u * SC_IBETA);
       const float sgn = sdf > 0.f ? 1.f : (sdf < 0.f ? -1.f : 0.f);
@@ -1071,7 +1074,7 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
       chain_layer(IC<2>{}, bias_s(lid_color + 2), TL.a_f2, TL.m_col[2]);
       // rgb.0 on (base + colour features), then rgb.2 + sigmoid
       wait_all();
-      {
+      if (lead) {
         const uint32_t b0 = bias_s(lid_rgb0), w2 = cblk_s + 4u * CL.rgb2_w, wd = cblk_s + 4u * CL.dir_w;
         float a0 = 0.f, a1 = 0.f, a2 = 0.f;
 #pragma unroll 1
@@ -1116,14 +1119,6 @@ __global__ void __launch_bounds__(kThreads, 1) field_fwd_kernel(const __grid_con
         st3(p.out.rgb, 1.f / (1.f + __expf(-a0)), 1.f / (1.f + __expf(-a1)), 1.f / (1.f + __expf(-a2)));
       }
     }
-    if constexpr (kProxy) {
-      if (g == 0) {  // tell the tape writers to leave
-        proxy_wait();
-        if (gtid == 0) proxy_cmd[1] = -1;
-        __syncwarp();
-        if (lane == 0) mbar_arrive(act_ready);
-      }
-    }
   }
 
   tc_fence_before_sync();
@@ -1139,7 +1134,8 @@ template <class Op, int B, int LMAX, bool DENSE, int WIDTH, bool SPLIT, bool SAV
 static cudaError_t launch_one(const FieldKernelParams& p, int n_sm, cudaStream_t stream) {
   auto kern = field_fwd_kernel<Op, B, LMAX, DENSE, WIDTH, SPLIT, SAVE>;
   constexpr int kPer = SPLIT ? 1 : 2;  // tiles in flight per CTA
-  const int smem = 1024 + kSmemArena + kSmemRing + (p.prog.cl.n_floats + kGroups * p.prog.fl.n_floats) * 4 + 256;
+  const int smem = 1024 + kSmemArena + kSmemRing + (p.prog.cl.n_floats + kGroups * p.prog.fl.n_floats) * 4 + kBarBytes +
+                   (SPLIT ? kSdfPartBytes : 0);
   if (smem > 227 * 1024) return cudaErrorInvalidValue;
   cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return e;

@@ -128,6 +128,10 @@ __device__ __forceinline__ void cluster_sync_all() {
 __device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
+// producer side of a named barrier: signals (releasing this thread's prior writes) without waiting
+__device__ __forceinline__ void named_bar_arrive(uint32_t id, uint32_t nthreads) {
+  asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
+}
 
 // one elected lane of a converged warp (elect.sync); cheaper for the issuing warp than `lane == 0`
 // predication: tools/mma_probe.cu measures 67 vs 102 cycles per N=128 MMA on B200
